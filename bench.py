@@ -6,7 +6,7 @@ channels, K=3 classes, 100 EM iterations per fit, synthetic complex128 STFT
 (iid complex Gaussian, seed 0) and an explicit seeded initialisation.
 One "step" = one complete fit (100 EM iterations) of one utterance.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 N > 1 (torchrun, one rank per GPU): every rank fits its own utterance of the
 same shape (the path shards over independent utterances / bins without any
@@ -305,6 +305,24 @@ def c3_bin_sharded_block(world, rank, barrier, reps=5):
     }
 
 
+def dump_outputs(model, out_dir):
+    """Writes the model of one timed step, as a caller of CACGMMTrainer.fit receives it, to out_dir/<name>.npy in
+    float64 (3.3 MB for C2).  Complex arrays get a trailing (real, imag) axis.  The eigenvectors carry an arbitrary
+    phase per column; the covariance V diag(lambda) V^H does not, so two builds can be compared on it."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        'weight': model.weight,                                                    # (F, K, 1)
+        'covariance_eigenvalues': model.cacg.covariance_eigenvalues,               # (F, K, D)
+        'covariance_eigenvectors': model.cacg.covariance_eigenvectors,             # (F, K, D, D, 2)
+        'covariance': model.cacg.covariance,                                       # (F, K, D, D, 2)
+    }
+    for name, t in arrays.items():
+        if t.is_complex():
+            t = torch.view_as_real(t)
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float64, copy=False))
+
+
 # --------------------------------------------------------------------------
 # B200 arm
 # --------------------------------------------------------------------------
@@ -368,11 +386,13 @@ def b200_arm(args):
             for e0, e1 in evs:
                 flush.fill_(1)
                 e0.record()
-                step_resident()
+                model = step_resident()
                 e1.record()
         barrier()
         launches = lib.pbb_launch_count() - launches0
     t_dev = sum(e0.elapsed_time(e1) for e0, e1 in evs) * 1e-3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(model, args.dump_outputs)
     # end to end through the public API with host buffers
     step_e2e()
     barrier()
@@ -508,7 +528,14 @@ def main():
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the model fitted in the last timed step to DIR/<name>.npy (float64, rank 0); the '
+                         'inputs are seeded, so runs with the same arguments can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200 (the reference arm keeps its models in the worker processes)')
     if args.impl == 'reference':
         reference_arm(args)
     else:

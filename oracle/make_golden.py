@@ -5,9 +5,11 @@ Run in the build container only (the GPU box has no reference checkout):
     PYTHONDONTWRITEBYTECODE=1 python -m oracle.make_golden
 
 Every fixture stores the inputs next to the reference's outputs, so the tests
-need neither the reference nor this script.  Quantities with an arbitrary
-phase / sign (eigenvectors, beamforming vectors, Watson modes) are stored as
-produced AND compared phase-invariantly by the tests.
+need neither the reference nor this script; the full-size and deflationSeed
+fixtures, which would pass 1 MB with them, store outputs only and the tests
+regenerate their inputs from the seeded generators of oracle/synth.py.
+Quantities with an arbitrary phase / sign (eigenvectors, beamforming vectors,
+Watson modes) are stored as produced AND compared phase-invariantly by the tests.
 """
 import os
 
@@ -307,7 +309,9 @@ def make_bf_wrapper(ref):
 
 def make_full_size(ref):
     """BASELINE.json configs 2 and 4 at FULL size, outputs only (the seeded inputs are regenerated by the tests):
-    the fitted model on every bin and the affiliations of every bin at every 8th frame."""
+    the fitted model on every bin and the affiliations of every bin at every 8th frame.  Every fixture file stays
+    below 1 MB: the model and the affiliations go to separate files, and the Hermitian covariance is stored as its
+    upper triangle (np.triu_indices order, diagonal included)."""
     T = ref.distribution.CACGMMTrainer
     for name, gen in (('c2_full_noise', lambda: synth.noise_stft(513, 500, 8, seed=0)),
                       ('c2_full_structured', lambda: synth.structured_stft(513, 500, 8, 3, seed=21)[0])):
@@ -315,19 +319,22 @@ def make_full_size(ref):
         init = synth.init_affiliation(513, 3, 500, seed=7)
         model = T().fit(y, initialization=init, iterations=100)
         aff = model.predict(y)
+        cov = model.cacg.covariance
+        iu = np.triu_indices(cov.shape[-1])
         np.savez_compressed(
             os.path.join(OUT, name + '.npz'), iterations=100,
             weight=model.weight, eigenvalues=model.cacg.covariance_eigenvalues,
-            covariance=model.cacg.covariance, affiliation_8=aff[..., ::8],
+            covariance_triu=cov[..., iu[0], iu[1]],
             log_likelihood=model.log_likelihood(y))
+        np.savez_compressed(os.path.join(OUT, name + '_affiliation.npz'), affiliation_8=aff[..., ::8])
     y = synth.noise_stft(257, 1000, 6, seed=4)
     init = synth.init_affiliation(257, 4, 1000, seed=7)
     model = ref.distribution.CWMMTrainer().fit(y, initialization=init, iterations=50)
     aff = model.predict(y)
     np.savez_compressed(
         os.path.join(OUT, 'c4_full_noise.npz'), iterations=50, weight=model.weight,
-        mode=model.complex_watson.mode, concentration=model.complex_watson.concentration,
-        affiliation_8=aff[..., ::8])
+        mode=model.complex_watson.mode, concentration=model.complex_watson.concentration)
+    np.savez_compressed(os.path.join(OUT, 'c4_full_noise_affiliation.npz'), affiliation_8=aff[..., ::8])
 
 
 def make_gcacgmm(ref):
@@ -389,12 +396,11 @@ def make_initializer(ref):
     out['dirichlet_a3'] = np.array(RI.iid.dirichlet(np.ones([2, 7, 3]), 3, alpha=3))
     out['flag_2'] = np.array(RI.deterministic.flag(Y, 2, permutation_free=True))
     out['flag_4_min'] = np.array(RI.deterministic.flag(np.ones([1, 5, 3]), 4, minimum=0.1, permutation_free=True))
+    # the inputs are not stored (the file would pass 1 MB): the test regenerates them from the same seeds
     y = synth.structured_stft(257, 60, 4, 3, seed=17)[0]
-    out['deflation_y'] = y
     out['deflation_pf'] = RI.deflation.deflationSeed(y, 3, permutation_free=True)
     out['deflation_nopf'] = RI.deflation.deflationSeed(y, 3, permutation_free=False, neighbors=3)
     sal = np.random.RandomState(2).uniform(0.1, 1, size=(257, 60))
-    out['deflation_sal'] = sal
     out['deflation_with_sal'] = RI.deflation.deflationSeed(y, 2, saliencies=sal, eps=1e-3)
     np.savez_compressed(os.path.join(OUT, 'initializer.npz'), **out)
 

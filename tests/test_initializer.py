@@ -39,14 +39,17 @@ def test_flag_initialiser():
 
 @pytest.mark.gpu
 def test_deflation_seed_matches_reference():
+    from oracle import synth
     from pb_bss_b200.initializer import deflation
-    y = GOLD['deflation_y']
+    # the inputs of oracle/make_golden.py: make_initializer, regenerated from the same seeds
+    y = synth.structured_stft(257, 60, 4, 3, seed=17)[0]
+    sal = np.random.RandomState(2).uniform(0.1, 1, size=(257, 60))
     got = deflation.deflationSeed(y, 3, permutation_free=True)
     assert got.shape == (3, 257, 60)
     np.testing.assert_allclose(got, GOLD['deflation_pf'], rtol=1e-9, atol=1e-12)
     np.testing.assert_allclose(deflation.deflationSeed(y, 3, permutation_free=False, neighbors=3),
                                GOLD['deflation_nopf'], rtol=1e-9, atol=1e-12)
-    np.testing.assert_allclose(deflation.deflationSeed(y, 2, saliencies=GOLD['deflation_sal'], eps=1e-3),
+    np.testing.assert_allclose(deflation.deflationSeed(y, 2, saliencies=sal, eps=1e-3),
                                GOLD['deflation_with_sal'], rtol=1e-9, atol=1e-12)
     np.testing.assert_allclose(got.sum(0), 1, atol=1e-12)
     import torch
